@@ -2,6 +2,7 @@
 """bench.py - KITTI-shape frames/s of the Point-GNN message-passing hot path on B200.
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--precision P]
+                    [--dump-outputs DIR]
 
 A *step* is one pass of the hot path (GPU graph construction + car_auto_T3 forward, real
 trained weights) over one batch of synthetic 20k-point KITTI-crop frames per GPU.  One JSON line is
@@ -299,7 +300,9 @@ def run_gpu(args, rank, world):
             torch.cuda.synchronize()
             stage_ms['gen graph'] += ev[0].elapsed_time(ev[1])
             stage_ms['gnn inference'] += ev[1].elapsed_time(ev[2])
-        return probs, boxes, kp[0].shape[0], edges[0].shape[0], edges[1].shape[0]
+        outputs = {'probs': probs, 'boxes': boxes, 'keypoint_indices': kp[0], 'keypoint_xyz': coords[1],
+                   'edges0': edges[0], 'edges1': edges[1]}
+        return probs, boxes, kp[0].shape[0], edges[0].shape[0], edges[1].shape[0], outputs
 
     # end-to-end arm: pinned host buffers on both sides (inputs above; outputs here, sized for the worst case of
     # one keypoint per point), asynchronous copies on the compute stream, ONE synchronisation per step
@@ -311,7 +314,7 @@ def run_gpu(args, rank, world):
         xyz = hx.to(dev, non_blocking=True)
         inten = hi.to(dev, non_blocking=True)
         fp = hfp.to(dev, non_blocking=True)
-        probs, boxes, k, e0, e1 = step_device(xyz, inten, fp)
+        probs, boxes, k, e0, e1, _ = step_device(xyz, inten, fp)
         hp, hb = out_probs[:k], out_boxes[:k]
         hp.copy_(probs, non_blocking=True)
         hb.copy_(boxes, non_blocking=True)
@@ -370,7 +373,7 @@ def run_gpu(args, rank, world):
         a = torch.cuda.Event(enable_timing=True)
         b = torch.cuda.Event(enable_timing=True)
         a.record()
-        probs, boxes, k, e0, e1 = step_device(*dev_steps[(args.warmup + s) % pool])
+        probs, boxes, k, e0, e1, outputs = step_device(*dev_steps[(args.warmup + s) % pool])
         b.record()
         b.synchronize()
         elapsed_ms += a.elapsed_time(b)
@@ -378,9 +381,14 @@ def run_gpu(args, rank, world):
         counters['keypoints'] += k
         counters['edges0'] += e0
         counters['edges1'] += e1
+        if s + 1 < args.steps:
+            outputs = None          # the graph of step s is not kept alive while step s + 1 allocates its own
     barrier()
     t_wall1 = time.perf_counter()
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
+    del outputs
 
     # ---- timed: end to end through the public API with host buffers ---------------------------
     barrier()
@@ -504,6 +512,27 @@ def run_gpu(args, rank, world):
         dist.destroy_process_group()
 
 
+DUMP_MAX_ARRAY_BYTES = 8 << 20     # 6 arrays: at most 48 MB written
+
+
+def dump_outputs(out_dir, outputs):
+    """Write what one timed step returned as <out_dir>/<name>.npy: floating point as float32 / float64, integer
+    indices as float64 (exact).  An array larger than DUMP_MAX_ARRAY_BYTES is replaced by a fixed sample of its rows
+    (seed 0, ascending row order; the edge lists at the default workload); <name>_rows.npy then holds the sampled row
+    numbers, so two builds that return the same number of rows are compared on the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        a = np.ascontiguousarray(t.detach().cpu().numpy())
+        a = a.astype(np.float64 if a.dtype.kind in 'iu' or a.dtype == np.float64 else np.float32)
+        row_bytes = a[:1].nbytes or 1
+        if a.nbytes > DUMP_MAX_ARRAY_BYTES:
+            m = DUMP_MAX_ARRAY_BYTES // (row_bytes + 8)
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], m, replace=False))
+            a = a[rows]
+            np.save(os.path.join(out_dir, name + '_rows.npy'), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def graph_roofline(ms, n, k, e0, e1, hbm, hbm_src):
     b = (n * 12 + k * 4) + (n * 12 + k * 12 + 4 * (k + 1) + 8 * e0) + (k * 12 + k * 12 + 4 * (k + 1) + 8 * e1)
     achieved = b / (ms * 1e-3) / 1e9 if ms > 0 else None
@@ -585,7 +614,13 @@ def main():
     ap.add_argument('--precision', default=None, choices=['fp32', 'bf16x3'])
     ap.add_argument('--frames-per-step', type=int, default=0)
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the outputs of the last one as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of the GPU path (--impl ours)')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))

@@ -20,8 +20,9 @@ installed here, so this module
 
 The variables (``VariableV2`` nodes) are read from the checkpoint's data file by
 name.  Used by tools/make_golden.py to produce tests/golden/gnn_*.npz and by
-tests/test_graphdef_cpu.py (live, when /root/reference is present) to pin
-oracle/gnn.py - and through it the CUDA path - to the reference.
+tests/test_graphdef_cpu.py (on the forward sub-graphs kept under
+tests/golden/checkpoints/) to pin oracle/gnn.py - and through it the CUDA path -
+to the reference.
 """
 import struct
 

@@ -1,8 +1,7 @@
-"""Run the reference's OWN models/graph_gen.py (build container only).
+"""Run the reference's OWN models/graph_gen.py (where the reference tree is present).
 
-TEST INFRASTRUCTURE.  /root/reference does not exist on the GPU box, so this
-module is only used by tools/make_golden.py (fixture generation) and by CPU
-tests that are skipped when the reference tree is absent.  graph_gen.py imports
+TEST INFRASTRUCTURE, used only by tools/make_golden.py to generate fixtures: the
+tests read what it computed from tests/golden/.  graph_gen.py imports
 ``open3d`` and ``tensorflow`` at module top (graph_gen.py:8-9) but uses neither
 in the radius-graph builder; empty stub modules make the import succeed.
 """
@@ -12,10 +11,6 @@ import sys
 import types
 
 REFERENCE_ROOT = '/root/reference'
-
-
-def available():
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, 'models', 'graph_gen.py'))
 
 
 def load():

@@ -57,3 +57,25 @@ def test_committed_bench_line_has_the_contract_keys():
         assert key in d['roofline'], key
     assert d['e2e']['h2d_bytes_per_step'] > 0 and d['e2e']['d2h_bytes_per_step'] > 0
     assert d['gpu_launches'] > 0 and d['warmup'] >= 3
+
+
+def test_dump_outputs_float_arrays_fixed_sample(tmp_path):
+    """--dump-outputs: float32 / float64 .npy files, integer indices exact, a large array replaced by the same seeded
+    sample of rows on every run, within the 64 MB budget."""
+    import numpy as np
+    import torch
+    bench = _bench()
+    edges = torch.arange(2 * 3000000, dtype=torch.int32).reshape(3000000, 2)
+    probs = torch.rand(1000, 4)
+    for run in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / run), {'probs': probs, 'edges1': edges})
+    files = sorted(os.listdir(tmp_path / 'a'))
+    assert files == ['edges1.npy', 'edges1_rows.npy', 'probs.npy']
+    assert sum(os.path.getsize(tmp_path / 'a' / f) for f in files) <= 64 << 20
+    for f in files:
+        a, b = np.load(tmp_path / 'a' / f), np.load(tmp_path / 'b' / f)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b)
+    assert np.array_equal(np.load(tmp_path / 'a' / 'probs.npy'), probs.numpy())
+    rows = np.load(tmp_path / 'a' / 'edges1_rows.npy').astype(np.int64)
+    assert 0 < len(rows) < 3000000 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(np.load(tmp_path / 'a' / 'edges1.npy'), edges.numpy()[rows].astype(np.float64))

@@ -7,7 +7,8 @@ weights (tools/make_golden.py).  Here:
 * oracle/gnn.py (the restatement every GPU parity test uses as its checker) must reproduce those
   vectors to 1e-5 for all seven shipped checkpoints,
 * a restatement with a swapped concat / subtraction order must NOT (the vectors discriminate),
-* when /root/reference is present the saved graph is re-interpreted live and must equal the fixtures.
+* the forward part of two saved graphs (tests/golden/checkpoints/, with the checkpoints rebuilt byte for byte by
+  oracle/golden_checkpoint.py) is re-interpreted and must equal the fixtures.
 """
 import glob
 import json
@@ -20,9 +21,6 @@ import pytest
 from conftest import ALL_CHECKPOINTS, GOLDEN, load_golden
 from oracle import gnn as ognn
 from oracle import graphdef
-
-REFERENCE = '/root/reference'
-
 
 def _v(n):
     out = b''
@@ -39,7 +37,7 @@ def _ld(num, payload):
     return _v(num << 3 | 2) + _v(len(payload)) + payload
 
 
-def test_wire_reader_decodes_nodedef():
+def test_wire_reader_decodes_nodedef(tmp_path):
     # TensorProto{dtype=DT_FLOAT, shape=[2,2], tensor_content}
     shape = _ld(2, _v(1 << 3) + _v(2)) + _ld(2, _v(1 << 3) + _v(2))
     tensor = _v(1 << 3) + _v(1) + _ld(2, shape) + _ld(4, struct.pack('<4f', 1, 2, 3, 4))
@@ -48,7 +46,7 @@ def test_wire_reader_decodes_nodedef():
     node = (_ld(1, b'scope/op') + _ld(2, b'Const') + _ld(3, b'a:1') + _ld(3, b'^ctl')
             + _ld(5, _ld(1, b'value') + _ld(2, attr_value)) + _ld(5, _ld(1, b'axis') + _ld(2, attr_i)))
     meta = _ld(2, _ld(1, node))                                   # MetaGraphDef.graph_def.node
-    path = os.path.join(os.environ.get('TMPDIR', '/tmp'), 'pg_test_meta.pb')
+    path = str(tmp_path / 'meta.pb')
     with open(path, 'wb') as f:
         f.write(meta)
     nodes = graphdef.load_meta_graph(path)
@@ -111,16 +109,20 @@ def test_fixtures_discriminate_operand_order(monkeypatch):
     assert np.abs(logits - g.gnn['logits']).max() > 0.1
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason='reference tree not present (GPU box)')
 @pytest.mark.parametrize('name', ['car_auto_T1_train', 'car_fixed_T3_train'])
-def test_live_saved_graph_equals_fixture(name):
+def test_live_saved_graph_equals_fixture(name, tmp_path):
+    from oracle import golden_checkpoint
     from pointgnn_b200.utils import tf_checkpoint
     g = load_golden(name)
-    ckpt = os.path.join(REFERENCE, 'checkpoints', name)
+    ckpt = golden_checkpoint.rebuild(name, str(tmp_path))
     meta = sorted(glob.glob(os.path.join(ckpt, 'model-*.meta')))[-1]
     coords, keypoints, edges = g.graph_tuple()
     out = graphdef.run_forward(meta, tf_checkpoint.load_checkpoint(ckpt), g.graph['intensity'], coords, keypoints,
                                edges)
     assert np.array_equal(out['logits'], g.gnn['logits']) and np.array_equal(out['boxes'], g.gnn['boxes'])
-    # the saved graph really is the full training graph (forward + loss + gradients), not a toy
-    assert len(graphdef.load_meta_graph(meta)) > 5000
+    # the sub-graph is cut from the full training graph (forward + loss + gradients), not a toy, and executes the
+    # same ops as the full graph did
+    with open(os.path.join(GOLDEN, 'graphdef_ops_%s.json' % name)) as f:
+        full = json.load(f)
+    assert full['meta'] == os.path.basename(meta) and full['nodes_total'] > 5000
+    assert out['ops'] == full['ops_executed']

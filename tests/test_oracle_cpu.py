@@ -1,9 +1,13 @@
-"""CPU tests: the oracle against the committed golden vectors and (when the build container's
-reference tree is present) against the reference's own graph_gen.py run live."""
+"""CPU tests: the oracle against the committed golden vectors, which hold what the reference's own code computed
+(tools/make_golden.py)."""
+import os
+
 import numpy as np
 import pytest
 
-from oracle import gnn, graph, reference_graph, synth
+from oracle import gnn, graph, synth
+
+GOLDEN = os.path.join(os.path.dirname(__file__), 'golden')
 
 
 def test_synth_is_seeded_and_kitti_shaped():
@@ -65,22 +69,23 @@ def test_voxel_keys_canonical_order():
     assert np.array_equal(np.sort(np.unique(keys)), ck[len(xyz):])
 
 
-@pytest.mark.skipif(not reference_graph.available(), reason='/root/reference only exists in the build container')
 def test_oracle_against_live_reference_graph_gen():
-    ref = reference_graph.load()
-    xyz, _ = synth.lidar_frame(11, 2500)
-    for voxel, r0, r1 in ((0.4, 1.0, 4.0), (0.2, 0.4, 1.6)):
+    """tests/golden/graph_live.npz: the edge lists the reference's own gen_disjointed_rnn_local_graph_v3 returned, and
+    scikit-learn's kd-tree 1-NN of the voxel centroids, on one frame at two scales."""
+    g = np.load(os.path.join(GOLDEN, 'graph_live.npz'))
+    xyz = g['xyz']
+    for i in range(2):
+        voxel, r0, r1 = (float(v) for v in g['params_%d' % i])
         cent = graph.voxel_down_sample(xyz, voxel)
         kp = graph.nearest_point(xyz, cent)
         kxyz = xyz[kp]
-        for pts, ctr, r in ((xyz, kxyz, r0), (kxyz, kxyz, r1)):
-            e_ref = ref.gen_disjointed_rnn_local_graph_v3(pts, ctr, r, -1)
+        for lvl, (pts, ctr, r) in enumerate(((xyz, kxyz, r0), (kxyz, kxyz, r1))):
+            e_ref = g['edges_%d_%d' % (i, lvl)].astype(np.int64)
             assert np.array_equal(graph.canonical_edges(e_ref), graph.radius_graph(pts, ctr, r))
         # kd-tree snap: identical except on exact distance ties (two-point voxels), where the
         # oracle's rule is "lowest index" and sklearn's is traversal order
-        from sklearn.neighbors import NearestNeighbors
-        idx = NearestNeighbors(n_neighbors=1, algorithm='kd_tree', n_jobs=1).fit(xyz).kneighbors(
-            cent, return_distance=False)[:, 0]
+        idx = g['knn_%d' % i].astype(np.int64)
+        assert len(idx) == len(kp)
         diff = np.flatnonzero(idx != kp)
         x64 = xyz.astype(np.float64)
         for j in diff:
@@ -131,10 +136,11 @@ def test_batch_graphs_offsets(car):
     assert np.array_equal(bk[0][k:], keypoints[0] + n)
 
 
-@pytest.mark.skipif(not reference_graph.available(), reason='/root/reference only exists in the build container')
-def test_checkpoint_reader_matches_golden_weights(car):
+def test_checkpoint_reader_matches_golden_weights(car, tmp_path):
+    """The reference's car_auto_T3_train checkpoint, rebuilt byte for byte (oracle/golden_checkpoint.py)."""
+    from oracle import golden_checkpoint
     from pointgnn_b200.utils import tf_checkpoint
-    w = tf_checkpoint.load_checkpoint('/root/reference/checkpoints/car_auto_T3_train')
+    w = tf_checkpoint.load_checkpoint(golden_checkpoint.rebuild('car_auto_T3_train', str(tmp_path)))
     assert w['Variable'] == 1400000
     for k, v in car.weights.items():
         assert np.array_equal(w[k], v)
@@ -159,21 +165,20 @@ def test_cpu_reference_baseline_matches_oracle(car):
     assert np.abs(probs - gnn.postprocess(car.gnn['logits'])).max() < 1e-5
 
 
-@pytest.mark.skipif(not reference_graph.available(), reason='/root/reference only exists in the build container')
-def test_all_shipped_checkpoints_load_and_run_through_the_oracle():
-    """Every checkpoint the reference ships (T0..T3, fixed / auto offset, car / ped) parses with the TF-free reader,
-    names every variable its frozen config asks for, and runs through the oracle forward on a small graph -
-    i.e. the restatement covers all shipped layer stacks, not just the two golden configurations."""
+def test_all_shipped_checkpoints_load_and_run_through_the_oracle(tmp_path):
+    """Every checkpoint the reference ships (T0..T3, fixed / auto offset, car / ped; rebuilt byte for byte by
+    oracle/golden_checkpoint.py) parses with the TF-free reader, names every variable its frozen config asks for, and
+    runs through the oracle forward on a small graph - i.e. the restatement covers all shipped layer stacks, not just
+    the two golden configurations."""
     import json
-    import os
+    from oracle import golden_checkpoint
     from pointgnn_b200.utils import tf_checkpoint
-    root = os.path.join(reference_graph.REFERENCE_ROOT, 'checkpoints')
     xyz, inten = synth.lidar_frame(5, 1500)
     seen = 0
-    for name in sorted(os.listdir(root)):
-        with open(os.path.join(root, name, 'config')) as f:
+    for name in golden_checkpoint.names():
+        with open(os.path.join(GOLDEN, 'config_%s.json' % name)) as f:
             config = json.load(f)
-        w = tf_checkpoint.load_checkpoint(os.path.join(root, name))
+        w = tf_checkpoint.load_checkpoint(golden_checkpoint.rebuild(name, str(tmp_path / name)))
         coords, kp, edges = graph.gen_multi_level_local_graph_v3(xyz, **config['runtime_graph_gen_kwargs'])
         layers = config['model_kwargs']['layer_configs']
         logits, boxes = gnn.predict(w, layers, config['num_classes'], 7, inten, coords, kp, edges)

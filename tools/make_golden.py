@@ -331,8 +331,100 @@ def graph_rnd3d_goldens():
     np.savez_compressed(os.path.join(GOLDEN, 'graph_rnd3d.npz'), **out)
 
 
+def graph_live_goldens():
+    """tests/golden/graph_live.npz: the reference's OWN gen_disjointed_rnn_local_graph_v3 (rows as it returns them,
+    int16: the frame has 2500 points) on the voxel keypoints of a seeded frame at two scales, and scikit-learn's kd-tree
+    1-NN of the voxel centroids."""
+    from sklearn.neighbors import NearestNeighbors
+    ref = reference_graph.load()
+    xyz, _ = synth.lidar_frame(11, 2500)
+    out = {'xyz': xyz}
+    for i, (voxel, r0, r1) in enumerate(((0.4, 1.0, 4.0), (0.2, 0.4, 1.6))):
+        cent = graph.voxel_down_sample(xyz, voxel)
+        kxyz = xyz[graph.nearest_point(xyz, cent)]
+        for lvl, (pts, ctr, r) in enumerate(((xyz, kxyz, r0), (kxyz, kxyz, r1))):
+            out['edges_%d_%d' % (i, lvl)] = ref.gen_disjointed_rnn_local_graph_v3(pts, ctr, r, -1).astype(np.int16)
+        out['knn_%d' % i] = NearestNeighbors(n_neighbors=1, algorithm='kd_tree', n_jobs=1).fit(xyz).kneighbors(
+            cent, return_distance=False)[:, 0].astype(np.int32)
+        out['params_%d' % i] = np.asarray([voxel, r0, r1], dtype=np.float64)
+    np.savez_compressed(os.path.join(GOLDEN, 'graph_live.npz'), **out)
+
+
+def checkpoint_goldens():
+    """tests/golden/checkpoints/<cfg>/: each shipped checkpoint in a form small enough to commit - its `checkpoint`
+    state file and `.index` table verbatim, and data.json, the byte layout of its `.data` file (tensor name, offset,
+    size, the bytes of the non-weight tensors, sha256 of the whole file).  oracle/golden_checkpoint.py rebuilds the
+    `.data` file from weights_<cfg>.npz and checks the sha256.  For the checkpoints in FORWARD_META the `.meta` is
+    kept too (gzipped), cut down to the forward sub-graph oracle/graphdef.run_forward executes (plus every
+    placeholder)."""
+    import gzip
+    import hashlib
+    import shutil
+    for name in CONFIGS:
+        src = os.path.join(reference_graph.REFERENCE_ROOT, 'checkpoints', name)
+        dst = os.path.join(GOLDEN, 'checkpoints', name)
+        os.makedirs(dst, exist_ok=True)
+        prefix = tf_checkpoint.latest_checkpoint(src)
+        base = os.path.basename(prefix)
+        shutil.copyfile(os.path.join(src, 'checkpoint'), os.path.join(dst, 'checkpoint'))
+        shutil.copyfile(prefix + '.index', os.path.join(dst, base + '.index'))
+        with open(prefix + '.data-00000-of-00001', 'rb') as f:
+            blob = f.read()
+        weights = dict(np.load(os.path.join(GOLDEN, 'weights_%s.npz' % name)))
+        tensors, extra = [], {}
+        for key, e in sorted(tf_checkpoint.read_index(prefix + '.index').items(), key=lambda kv: kv[1]['offset']):
+            assert e['shard'] == 0
+            tensors.append([key, e['offset'], e['size']])
+            raw = blob[e['offset']:e['offset'] + e['size']]
+            if key in weights:
+                assert weights[key].astype('<f4').tobytes() == raw, key
+            else:
+                extra[key] = raw.hex()
+        layout = {'data_file': base + '.data-00000-of-00001', 'size': len(blob),
+                  'sha256': hashlib.sha256(blob).hexdigest(), 'tensors': tensors, 'extra_hex': extra}
+        with open(os.path.join(dst, 'data.json'), 'w') as f:
+            json.dump(layout, f, indent=0)
+        if name in FORWARD_META:
+            meta = sorted(glob.glob(os.path.join(src, 'model-*.meta')))[-1]
+            with gzip.open(os.path.join(dst, os.path.basename(meta) + '.gz'), 'wb') as f:
+                f.write(forward_meta_graph(meta))
+        print('checkpoint', name, len(tensors), 'tensors', sorted(extra))
+
+
+FORWARD_META = ('car_auto_T1_train', 'car_fixed_T3_train')
+
+
+def forward_meta_graph(meta_path):
+    """-> a MetaGraphDef (bytes) holding only the NodeDefs run_forward reads, each copied byte for byte."""
+    def ld(num, payload):
+        head, n = b'', len(payload)
+        tag = num << 3 | 2
+        for v in (tag, n):
+            while True:
+                b, v = v & 0x7F, v >> 7
+                head += bytes([b | 0x80]) if v else bytes([b])
+                if not v:
+                    break
+        return head + payload
+
+    nodes = graphdef.load_meta_graph(meta_path)
+    keep = graphdef._closure(nodes, [graphdef.LOGITS_NODE, graphdef.BOXES_NODE, graphdef.PROBS_NODE])
+    keep |= {n for n in nodes if nodes[n].op == 'Placeholder'}
+    with open(meta_path, 'rb') as f:
+        buf = memoryview(f.read())
+    body = b''
+    for num, _, val in graphdef.fields(buf):
+        if num == 2:
+            for n2, _, v2 in graphdef.fields(val):
+                if n2 == 1 and graphdef._node(v2).name in keep:
+                    body += ld(1, bytes(v2))
+    return ld(2, body)
+
+
 if __name__ == '__main__':
     which = sys.argv[1] if len(sys.argv) > 1 else 'all'
+    if which in ('all', 'graph_live'):
+        graph_live_goldens()
     if which in ('all', 'graph_random'):
         graph_random_goldens()
     if which in ('all', 'graph_multiscale'):
@@ -347,3 +439,5 @@ if __name__ == '__main__':
         post_goldens()
     if which in ('all', 'kitti'):
         kitti_goldens()
+    if which in ('all', 'checkpoints'):     # after 'gnn': rebuilt from the weights_<cfg>.npz it writes
+        checkpoint_goldens()
