@@ -222,16 +222,21 @@ PG_API int pg_multi_level_graph(const float* xyz, const int32_t* frame_ptr, int3
  * these two calls take their randomness as ARGUMENTS; everything else is reproduced exactly.
  *
  * pg_random_keypoints = multi_layer_downsampling_random for one scale (graph_gen.py:92-153):
- *   voxel index of every point: floor_divide(p - frame_min, voxel) in float32 (shift_host == NULL, add_rnd3d
- *   false, :124-126) or floor_divide(p - frame_min + voxel * shift, voxel) in float64 (:127-130), shift_host =
- *   (host) [num_frames][3] the np.random.random((1,3)) draw of each frame;
+ *   xyz / frame_ptr [num_points]: the ORIGINAL cloud, whose per-frame minimum frame_min is the grid origin of every
+ *   level (:107-110); base_xyz / base_frame_ptr [num_base]: the points voxelised at this scale, the previous level's
+ *   vertices (:115);
+ *   voxel index of every base point: floor_divide(p - frame_min, voxel) in float32 (shift_host == NULL, add_rnd3d
+ *   false and a scalar voxel size, :123-124) or floor_divide(p - frame_min + voxel * shift, voxel) in float64
+ *   (:126-128), shift_host = (host) [num_frames][3] the np.random.random((1,3)) draw of each frame; an all-zero
+ *   shift gives the float64 quotient NumPy computes for an array voxel size without add_rnd3d;
  *   one keypoint per occupied voxel, voxels in order of first appearance (the dict order of :133-139);
- *   keypoint o = the floor(uniform[o] * count)-th point (ascending index) of its voxel - uniform [capacity]
+ *   keypoint o = the floor(uniform[o] * count)-th point (ascending index) of its voxel - uniform [num_base]
  *   device fp32 in [0,1) stands in for random.choice (:143-146).
- * Outputs as pg_voxel_keypoints.
+ * Outputs as pg_voxel_keypoints: out_keypoint_idx [K] rows of base_xyz.
  */
 PG_API int pg_random_keypoints(const float* xyz, const int32_t* frame_ptr, int32_t num_frames,
                         int64_t num_points, const double* voxel_size_host, const double* shift_host,
+                        const float* base_xyz, const int32_t* base_frame_ptr, int64_t num_base,
                         const float* uniform, int32_t* out_keypoint_idx, int64_t capacity,
                         int32_t* out_kp_frame_ptr, int64_t* out_num_keypoints_host, void* stream);
 

@@ -262,6 +262,36 @@ def multi_layer_downsampling_random(points_xyz, base_voxel_size, levels=(1,), ad
     return vertex_coord_list, keypoint_indices_list
 
 
+RANDOM_GOLDEN_CASES = ('plain', 'rnd3d', 'ms_plain', 'ms_rnd3d', 'arr')
+
+
+def random_golden_case(g, tag):
+    """One case of tests/golden/graph_random.npz (written by tools/make_golden.py::graph_random_goldens) ->
+    dict(xyz, levels, voxel, add_rnd3d, shifts, uniforms, kp, coords, radii, edges).  shifts / uniforms / kp / coords
+    are per level (None where a level draws nothing); kp[i] indexes level i's input, coords[i] = level i + 1's vertices;
+    voxel is a Python float for a scalar voxel size and a float64 array for an array one; radii / edges: the radius
+    graph of each level where the case pins it, else None."""
+    files = set(g.files)
+    if tag in ('plain', 'rnd3d'):          # levels [1, 1], scalar voxel 0.8
+        add, xyz, kp0 = tag == 'rnd3d', g['xyz'], g['kp_' + tag]
+        return dict(xyz=xyz, levels=[1, 1], voxel=0.8, add_rnd3d=add,
+                    shifts=[g['shift_' + tag] if add else None, None], uniforms=[g['u_' + tag], None],
+                    kp=[kp0, np.arange(len(kp0))], coords=[xyz[kp0], xyz[kp0]], radii=None, edges=None)
+    levels = [float(v) for v in g['levels_' + tag]]
+    voxel = g['voxel_' + tag]
+
+    def per_level(kind, shift_by=0):
+        keys = ['%s_%s_%d' % (kind, tag, li + shift_by) for li in range(len(levels))]
+        return [g[k] if k in files else None for k in keys]
+    edges = None
+    if 'radii_' + tag in files:
+        edges = [g['edges_%s_%d' % (tag, lvl)] for lvl in range(len(g['radii_' + tag]))]
+    return dict(xyz=g['xyz_' + tag] if 'xyz_' + tag in files else g['xyz'], levels=levels,
+                voxel=float(voxel) if voxel.ndim == 0 else voxel, add_rnd3d=bool(g['add_' + tag]),
+                shifts=per_level('shift'), uniforms=per_level('u'), kp=per_level('kp'), coords=per_level('coords', 1),
+                radii=[float(r) for r in g['radii_' + tag]] if edges is not None else None, edges=edges)
+
+
 def check_neighbor_cap(full_edges, capped_edges, num_neighbors):
     """Invariants of graph_gen.py:210-214 that do not depend on the draw: per destination, rows of at most
     num_neighbors entries are unchanged, longer rows keep exactly num_neighbors DISTINCT members of the row."""

@@ -52,8 +52,8 @@ SIGNATURES = {
                                             c_i32p, c_i32p, c_i32p, c_i64, c_i32p, c_i32p, c_i32p, c_i64,
                                             ctypes.POINTER(c_i64), ctypes.c_void_p]),
     'pg_random_keypoints': (ctypes.c_int, [c_f32p, c_i32p, c_i32, c_i64, ctypes.POINTER(ctypes.c_double),
-                                           ctypes.POINTER(ctypes.c_double), c_f32p, c_i32p, c_i64, c_i32p,
-                                           ctypes.POINTER(c_i64), ctypes.c_void_p]),
+                                           ctypes.POINTER(ctypes.c_double), c_f32p, c_i32p, c_i64, c_f32p, c_i32p,
+                                           c_i64, c_i32p, ctypes.POINTER(c_i64), ctypes.c_void_p]),
     'pg_cap_neighbors': (ctypes.c_int, [c_i32p, c_i32p, c_i64, c_i32, ctypes.c_uint32, c_i32p, c_i32p, c_i32p, c_i64,
                                         ctypes.POINTER(c_i64), ctypes.c_void_p]),
     'pg_scatter_max': (ctypes.c_int, [c_f32p, c_i32p, c_i64, c_i32, c_i64, c_f32p, ctypes.c_void_p]),
@@ -234,13 +234,18 @@ def voxel_keypoints_rnd3d(xyz, frame_ptr, voxel_size, shift, base_xyz=None, base
     return (None if out_idx is None else out_idx[:k.value]), out_fp, (None if cent is None else cent[:k.value])
 
 
-def random_keypoints(xyz, frame_ptr, voxel_size, shift, uniform):
-    """pg_random_keypoints.  shift: None or [F,3] float64 host array; uniform: [N] CUDA fp32 in [0,1).
-    -> (keypoint_idx [K] int32, kp_frame_ptr [F+1] int32)."""
+def random_keypoints(xyz, frame_ptr, voxel_size, shift, base_xyz, base_frame_ptr, uniform):
+    """pg_random_keypoints.  xyz / frame_ptr: the original cloud (grid origin); base_xyz / base_frame_ptr: the points
+    voxelised; shift: None or [F,3] float64 host array; uniform: [len(base_xyz)] CUDA fp32 in [0,1).
+    -> (keypoint_idx [K] int32 rows of base_xyz, kp_frame_ptr [F+1] int32)."""
     import numpy as np
     lib = load()
-    n = xyz.shape[0]
+    n = base_xyz.shape[0]
     num_frames = frame_ptr.numel() - 1
+    if base_frame_ptr.numel() != num_frames + 1:
+        raise ValueError('base_frame_ptr has %d entries, expected %d' % (base_frame_ptr.numel(), num_frames + 1))
+    if uniform.numel() < n:
+        raise ValueError('uniform has %d entries, need one per base point (%d)' % (uniform.numel(), n))
     out_idx = torch.empty(n, dtype=torch.int32, device=xyz.device)
     out_fp = torch.empty(num_frames + 1, dtype=torch.int32, device=xyz.device)
     vs = (ctypes.c_double * 3)(*[float(v) for v in voxel_size])
@@ -250,7 +255,9 @@ def random_keypoints(xyz, frame_ptr, voxel_size, shift, uniform):
         sh = sh_arr.ctypes.data_as(ctypes.POINTER(ctypes.c_double))
     k = c_i64(0)
     _check(lib.pg_random_keypoints(_ptr(xyz, torch.float32, 'xyz'), _ptr(frame_ptr, torch.int32, 'frame_ptr'), num_frames,
-                                   n, vs, sh, _ptr(uniform, torch.float32, 'uniform'), _ptr(out_idx, torch.int32, 'out'), n,
+                                   xyz.shape[0], vs, sh, _ptr(base_xyz, torch.float32, 'base_xyz'),
+                                   _ptr(base_frame_ptr, torch.int32, 'base_frame_ptr'), n,
+                                   _ptr(uniform, torch.float32, 'uniform'), _ptr(out_idx, torch.int32, 'out'), n,
                                    _ptr(out_fp, torch.int32, 'out_fp'), ctypes.byref(k), _stream()))
     return out_idx[:k.value], out_fp
 

@@ -1135,7 +1135,8 @@ extern "C" int pg_multi_level_graph(const float* xyz, const int32_t* frame_ptr, 
 // Training-time graph path (SURVEY 8a-3 / 8f-4): random voxel keypoints and the random neighbour cap.
 // The reference draws from Python's / NumPy's global generators (graph_gen.py:92-153, 210-214), so parity is
 // statistical; everything that is NOT random is reproduced exactly: the voxel index arithmetic (float32
-// floor-division without the random shift, float64 with it), the set of occupied voxels, the first-appearance
+// floor-division for a scalar voxel size without the random shift, float64 with it or for an array voxel size; the
+// grid origin is the minimum of the original cloud at every level), the set of occupied voxels, the first-appearance
 // output order of the keypoints, "one point of its own voxel per keypoint", and for the cap "rows of at most
 // num_neighbors entries keep every neighbour, longer rows keep exactly num_neighbors distinct neighbours".
 // =================================================================================================
@@ -1171,14 +1172,19 @@ __device__ void shifted_cell_of(const GridSpec& g, const uint32_t* __restrict__ 
 }
 
 // graph_gen.py:124-131 voxel index of every point; shift == nullptr: float32 arithmetic (add_rnd3d False),
-// else float64 with the per-frame random shift fractions (add_rnd3d True)
+// else float64 with the per-frame random shift fractions (add_rnd3d True; a zero shift gives the exact float64
+// quotient of an array voxel size).  `bounds` holds the per-frame minimum of the ORIGINAL cloud (origin_frame_ptr,
+// num_origin rows), which fixes the grid origin of every level (graph_gen.py:107-110).
 __global__ void random_voxel_keys_kernel(const float* __restrict__ xyz, const int32_t* __restrict__ frame_ptr, int num_frames,
-                                         int64_t n, double vx, double vy, double vz, const double* __restrict__ shift,
+                                         int64_t n, const int32_t* __restrict__ origin_frame_ptr, int64_t num_origin,
+                                         double vx, double vy, double vz, const double* __restrict__ shift,
                                          const uint32_t* __restrict__ bounds, uint64_t* __restrict__ keys,
                                          int32_t* __restrict__ vals, int* __restrict__ err) {
   const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  if (i == 0 && (frame_ptr[0] != 0 || int64_t(frame_ptr[num_frames]) != n)) atomicOr(err, kErrFramePtr);
+  if (i == 0 && (frame_ptr[0] != 0 || int64_t(frame_ptr[num_frames]) != n || origin_frame_ptr[0] != 0 ||
+                 int64_t(origin_frame_ptr[num_frames]) != num_origin))
+    atomicOr(err, kErrFramePtr);
   const int f = find_frame(frame_ptr, num_frames, i);
   const float mn[3] = {ordered_to_float(bounds[3 * f]), ordered_to_float(bounds[3 * f + 1]), ordered_to_float(bounds[3 * f + 2])};
   const double v[3] = {vx, vy, vz};
@@ -1309,16 +1315,19 @@ __global__ void __launch_bounds__(256) cap_rows_kernel(const int32_t* __restrict
 }  // namespace pg
 
 extern "C" int pg_random_keypoints(const float* xyz, const int32_t* frame_ptr, int32_t num_frames, int64_t num_points,
-                                   const double* voxel_size_host, const double* shift_host, const float* uniform,
+                                   const double* voxel_size_host, const double* shift_host, const float* base_xyz,
+                                   const int32_t* base_frame_ptr, int64_t num_base, const float* uniform,
                                    int32_t* out_keypoint_idx, int64_t capacity, int32_t* out_kp_frame_ptr,
                                    int64_t* out_num_keypoints_host, void* stream) {
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  PG_REQUIRE(xyz && frame_ptr && voxel_size_host && uniform && out_keypoint_idx && out_kp_frame_ptr && out_num_keypoints_host,
+  PG_REQUIRE(xyz && frame_ptr && voxel_size_host && base_xyz && base_frame_ptr && uniform && out_keypoint_idx &&
+                 out_kp_frame_ptr && out_num_keypoints_host,
              "pg_random_keypoints: null argument");
   PG_REQUIRE(voxel_size_host[0] > 0 && voxel_size_host[1] > 0 && voxel_size_host[2] > 0, "voxel size must be positive");
   PG_REQUIRE(num_frames >= 1 && num_frames <= 65534, "num_frames=%d out of range [1,65534]", num_frames);
-  const int64_t n = num_points;
-  PG_REQUIRE(n >= 1 && n < (int64_t(1) << 31), "num_points=%lld out of range", (long long)n);
+  PG_REQUIRE(num_points >= 1 && num_points < (int64_t(1) << 31), "num_points=%lld out of range", (long long)num_points);
+  const int64_t n = num_base;      // the points that are voxelised; xyz only sets the grid origin
+  PG_REQUIRE(n >= 1 && n < (int64_t(1) << 31), "num_base=%lld out of range", (long long)n);
   Temp bounds, keys_a, keys_b, vals_a, vals_b, head, head_scan, cell_key, cell_start, keys2a, keys2b, vals2a, vals2b, tmp, err,
       shift;
   PG_CUDA_OK(bounds.alloc(sizeof(uint32_t) * 3 * num_frames, s));
@@ -1344,12 +1353,13 @@ extern "C" int pg_random_keypoints(const float* xyz, const int32_t* frame_ptr, i
   }
   init_bounds_kernel<<<ceil_div(3 * num_frames, 256), 256, 0, s>>>(bounds.as<uint32_t>(), 3 * num_frames);
   PG_LAUNCH_CHECK();
-  const int blocks_per_frame = int(std::min<int64_t>(std::max<int64_t>(1, ceil_div(n / num_frames, 1024)), 64));
-  frame_min_kernel<<<dim3(blocks_per_frame, num_frames), 256, 0, s>>>(xyz, frame_ptr, n, bounds.as<uint32_t>());
+  const int blocks_per_frame = int(std::min<int64_t>(std::max<int64_t>(1, ceil_div(num_points / num_frames, 1024)), 64));
+  frame_min_kernel<<<dim3(blocks_per_frame, num_frames), 256, 0, s>>>(xyz, frame_ptr, num_points, bounds.as<uint32_t>());
   PG_LAUNCH_CHECK();
-  random_voxel_keys_kernel<<<ceil_div(n, 256), 256, 0, s>>>(xyz, frame_ptr, num_frames, n, voxel_size_host[0], voxel_size_host[1],
-                                                            voxel_size_host[2], shift_dev, bounds.as<uint32_t>(),
-                                                            keys_a.as<uint64_t>(), vals_a.as<int32_t>(), err.as<int>());
+  random_voxel_keys_kernel<<<ceil_div(n, 256), 256, 0, s>>>(base_xyz, base_frame_ptr, num_frames, n, frame_ptr, num_points,
+                                                            voxel_size_host[0], voxel_size_host[1], voxel_size_host[2],
+                                                            shift_dev, bounds.as<uint32_t>(), keys_a.as<uint64_t>(),
+                                                            vals_a.as<int32_t>(), err.as<int>());
   PG_LAUNCH_CHECK();
   int frame_bits = 1;
   while ((1 << frame_bits) < num_frames + 1) ++frame_bits;

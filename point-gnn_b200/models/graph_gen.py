@@ -13,13 +13,20 @@ device).  Built: the deterministic inference path (``add_rnd3d=False``, ``downsa
 ``num_neighbors <= 0``) and the training-time path of train.py:88-90 with configs/*_train_config
 (``downsample_method='random'`` with or without ``add_rnd3d``, ``num_neighbors > 0``,
 graph_gen.py:92-153, 210-214).  The random path takes its randomness from NumPy's global generator for
-the per-frame grid shift - the same ``np.random.random((1, 3))`` draw as the reference - and from this
-module's CUDA generator (``set_seed``) for the per-voxel choice and the neighbour cap, where the
-reference uses Python's ``random`` / ``np.random.choice``: results are equal in distribution, not draw
-by draw.  ``add_rnd3d`` with the centroid method (graph_gen.py:24-39) draws the same ``np.random.random((1, 3))``
-per level; its centroids equal the reference's to float32 summation accuracy (the reference sums in float32 in
-``argsort`` order).  The per-axis ``scale`` of ``gen_disjointed_rnn_local_graph_v3`` (graph_gen.py:203-206) is
-divided in float64 inside the kernels, as ``points_xyz / np.array(scale)`` does.
+the per-frame grid shift - the same ``np.random.random((1, 3))`` draws as the reference, frame-major: a batch of
+F frames gets the draws of F one-frame calls - and from this module's CUDA generator (``set_seed``) for the
+per-voxel choice and the neighbour cap, where the reference uses Python's ``random`` / ``np.random.choice``:
+results are equal in distribution, not draw by draw.  Everything else is the reference's arithmetic: every level's
+grid starts at the minimum of the original cloud (graph_gen.py:107-110), and the voxel index is a float32
+floor-division for a scalar voxel size and float64 for an array one or with ``add_rnd3d``, as NumPy promotes.
+Given the same random numbers (``_downsampling_random(..., uniform=, shifts=)``) the keypoints are the reference's
+bit for bit (tests/test_graph_random_gpu.py against tests/golden/graph_random.npz).  A capped neighbour row keeps
+its members in ascending source order where the reference keeps ``np.random.choice``'s random order; the model
+only reduces a row with a segment max, which does not depend on the order.  ``add_rnd3d`` with the centroid method
+(graph_gen.py:24-39) draws the same ``np.random.random((1, 3))`` per frame and new scale; its centroids equal the
+reference's to float32 summation accuracy (the reference sums in float32 in ``argsort`` order).  The per-axis
+``scale`` of ``gen_disjointed_rnn_local_graph_v3`` (graph_gen.py:203-206) is divided in float64 inside the
+kernels, as ``points_xyz / np.array(scale)`` does.
 
 Extra, backwards-compatible keyword ``frame_ptr``: a [F+1] int array batching F frames in one
 call; the result is then exactly what the reference's ``batch_data`` (train.py:135-171) builds
@@ -82,6 +89,36 @@ def _voxel_vector(base_voxel_size, level):
     return np.broadcast_to(v, (3,)).astype(np.float64)
 
 
+def _divides_in_float64(base_voxel_size, level):
+    """graph_gen.py:123-124 floor-divides float32 coordinates by ``base_voxel_size*level``: NumPy keeps float32 for a
+    Python float and promotes to float64 for a float64 array (what gen_multi_level_local_graph_v3 makes of a list,
+    :172-173).  Probe the promotion instead of restating it."""
+    if isinstance(base_voxel_size, list):
+        base_voxel_size = np.array(base_voxel_size)
+    return (np.zeros((1, 3), dtype=np.float32) // (base_voxel_size * level)).dtype == np.float64
+
+
+def _new_scales(levels):
+    """Per level: True where it voxelises (a scale different from the previous level's), False for a repeated scale."""
+    flags, last_level = [], 0
+    for level in levels:
+        flags.append(not np.isclose(level, last_level))
+        last_level = level
+    return flags
+
+
+def _rnd3d_shifts(levels, num_frames):
+    """The add_rnd3d grid shifts of F frames, one np.random.random((1, 3)) per frame and new scale, drawn frame-major:
+    the reference builds one frame per call (train.py:88-90), and each call draws its scales in turn (graph_gen.py:24-27,
+    126-128), so frame f gets the draws F separate calls would give it.  -> per level: [F,3] float64 or None."""
+    new = [li for li, is_new in enumerate(_new_scales(levels)) if is_new]
+    draws = [[np.random.random((1, 3)) for _ in new] for _ in range(num_frames)]
+    shifts = [None] * len(levels)
+    for j, li in enumerate(new):
+        shifts[li] = np.vstack([draws[f][j] for f in range(num_frames)])
+    return shifts
+
+
 def multi_layer_downsampling(points_xyz, base_voxel_size, levels=[1], add_rnd3d=False):
     """graph_gen.py:11-47 (Open3D branch).  -> list: the cloud, then per level the fp64 voxel centroids of the
     ORIGINAL cloud at that scale (a level with the previous level's scale repeats the previous entry, :21-22).
@@ -121,10 +158,11 @@ def _downsampling_select(cloud, base_voxel_size, levels, add_rnd3d):
     vertex_coord_list = [cloud.xyz]
     frame_ptr_list = [cloud.frame_ptr]
     keypoint_indices_list = []
-    last_level = 0
-    for level in levels:
+    # graph_gen.py:24-39: random grid shift, one np.random.random((1, 3)) per frame and new scale (frame-major)
+    shifts = _rnd3d_shifts(levels, num_frames) if add_rnd3d else None
+    for li, (level, is_new) in enumerate(zip(levels, _new_scales(levels))):
         base_points = vertex_coord_list[-1]
-        if np.isclose(level, last_level):
+        if not is_new:
             # same scale (a gnn layer): identity, graph_gen.py:76-81
             vertex_coord_list.append(base_points)
             frame_ptr_list.append(frame_ptr_list[-1])
@@ -135,10 +173,7 @@ def _downsampling_select(cloud, base_voxel_size, levels, add_rnd3d):
             # graph_gen.py:41-45 voxelises the ORIGINAL cloud, :84-88 snaps to the previous level.
             voxel = _voxel_vector(base_voxel_size, level)
             if add_rnd3d:
-                # graph_gen.py:24-39: random grid shift, one np.random.random((1, 3)) per frame and level (each
-                # fetch_data call of the reference draws its own)
-                shift = np.vstack([np.random.random((1, 3)) for _ in range(num_frames)])
-                idx, kp_fp, _ = _lib.voxel_keypoints_rnd3d(cloud.xyz, cloud.frame_ptr, voxel, shift, base_points,
+                idx, kp_fp, _ = _lib.voxel_keypoints_rnd3d(cloud.xyz, cloud.frame_ptr, voxel, shifts[li], base_points,
                                                            frame_ptr_list[-1])
             elif base_points is cloud.xyz:
                 # every shipped config: one distinct scale, previous level == original cloud (one grid, one kernel)
@@ -152,7 +187,6 @@ def _downsampling_select(cloud, base_voxel_size, levels, add_rnd3d):
             kidx = idx[:, None]
             kidx._pg_trusted = (int(base_points.shape[0]), kidx._version)    # rows of the level it was snapped to
             keypoint_indices_list.append(kidx)
-        last_level = level
     return vertex_coord_list, keypoint_indices_list, frame_ptr_list
 
 
@@ -168,36 +202,40 @@ def multi_layer_downsampling_random(points_xyz, base_voxel_size, levels=[1], add
 
 def _downsampling_random(cloud, base_voxel_size, levels, add_rnd3d, uniform=None, shifts=None):
     """Device-side body of multi_layer_downsampling_random.  ``uniform`` / ``shifts`` (tests): explicit random
-    numbers instead of draws from the generators."""
+    numbers per level instead of draws from the generators - ``uniform[li]`` one float32 in [0,1) per voxel of level li
+    in first-appearance order (at least one per point of the previous level), ``shifts[li]`` the [F,3] grid shifts."""
     vertex_coord_list = [cloud.xyz]
     frame_ptr_list = [cloud.frame_ptr]
     keypoint_indices_list = []
-    last_level = 0
     num_frames = cloud.frame_ptr.numel() - 1
-    for li, level in enumerate(levels):
+    if add_rnd3d and shifts is None:
+        shifts = _rnd3d_shifts(levels, num_frames)
+    for li, (level, is_new) in enumerate(zip(levels, _new_scales(levels))):
         base_points = vertex_coord_list[-1]
-        if np.isclose(level, last_level):
+        if not is_new:
             vertex_coord_list.append(base_points)
             frame_ptr_list.append(frame_ptr_list[-1])
             kidx = torch.arange(base_points.shape[0], dtype=torch.int32, device=base_points.device)[:, None]
             kidx._pg_trusted = (int(base_points.shape[0]), kidx._version)
             keypoint_indices_list.append(kidx)
         else:
-            # graph_gen.py:115: the PREVIOUS level is voxelised (not the original cloud as in the centroid method)
-            shift = None
-            if add_rnd3d:       # one np.random.random((1, 3)) per frame, as each fetch_data call draws (train.py:88-90)
-                shift = shifts[li] if shifts is not None else np.vstack(
-                    [np.random.random((1, 3)) for _ in range(num_frames)])
+            # graph_gen.py:115: the PREVIOUS level is voxelised (not the original cloud as in the centroid method), on the
+            # grid whose origin is the minimum of the ORIGINAL cloud (:107-110) at every level
+            if add_rnd3d:
+                shift = shifts[li]
+            elif _divides_in_float64(base_voxel_size, level):
+                shift = np.zeros((num_frames, 3))       # a zero shift takes the kernel's exact float64 quotient
+            else:
+                shift = None
             u = uniform[li] if uniform is not None else torch.rand(base_points.shape[0], generator=_generator(),
                                                                    device=base_points.device, dtype=torch.float32)
-            idx, kp_fp = _lib.random_keypoints(base_points, frame_ptr_list[-1], _voxel_vector(base_voxel_size, level),
-                                               shift, u)
+            idx, kp_fp = _lib.random_keypoints(cloud.xyz, cloud.frame_ptr, _voxel_vector(base_voxel_size, level), shift,
+                                               base_points, frame_ptr_list[-1], u)
             vertex_coord_list.append(_lib.gather_rows(base_points, idx))
             frame_ptr_list.append(kp_fp)
             kidx = idx[:, None]
             kidx._pg_trusted = (int(base_points.shape[0]), kidx._version)
             keypoint_indices_list.append(kidx)
-        last_level = level
     return vertex_coord_list, keypoint_indices_list, frame_ptr_list
 
 

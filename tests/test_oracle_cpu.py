@@ -236,3 +236,81 @@ def test_oracle_rnd3d_centroids_match_reference_golden():
         assert np.array_equal(np.asarray(cents[i + 1], dtype=np.float64), g['centroids_%d' % (i + 1)])
         assert (kp[i][:, 0] == g['kp_%d' % i]).mean() > 0.97
     assert np.array_equal(kp[1][:, 0], np.arange(len(kp[0])))
+
+
+@pytest.mark.parametrize('tag', graph.RANDOM_GOLDEN_CASES)
+def test_oracle_random_downsampling_matches_reference_golden(tag):
+    """The training-time keypoint choice (graph_gen.py:92-153): tests/golden/graph_random.npz holds the reference's own
+    multi_layer_downsampling_random with its random sources patched to recorded numbers.  Fed the same numbers, the
+    oracle's restatement must return the same keypoints and vertices - at a repeated scale, at a second distinct scale
+    (grid origin = the ORIGINAL cloud's minimum) and with an array voxel size (float64 floor-division)."""
+    c = graph.random_golden_case(np.load(os.path.join(GOLDEN, 'graph_random.npz')), tag)
+    coords, kp = graph.multi_layer_downsampling_random(c['xyz'], c['voxel'], c['levels'], c['add_rnd3d'],
+                                                       shifts=c['shifts'], uniforms=c['uniforms'])
+    assert len(kp) == len(c['levels'])
+    for li in range(len(c['levels'])):
+        assert np.array_equal(kp[li][:, 0], c['kp'][li]), li
+        assert coords[li + 1].dtype == np.float32 and np.array_equal(coords[li + 1], c['coords'][li]), li
+    if c['edges'] is not None:
+        for lvl, r in enumerate(c['radii']):
+            assert np.array_equal(graph.radius_graph(coords[lvl], coords[lvl + 1], r), c['edges'][lvl]), lvl
+
+
+def test_random_golden_discriminates_the_divergences():
+    """The fixture's cases would catch a grid origin taken from the previous level and a float32 division for an array
+    voxel size: those rules give different keypoints on the same recorded numbers."""
+    g = np.load(os.path.join(GOLDEN, 'graph_random.npz'))
+    for tag in ('ms_plain', 'ms_rnd3d'):
+        c = graph.random_golden_case(g, tag)
+        li = 1                                  # the second scale, voxelised on its own minimum
+        _, kp = graph.multi_layer_downsampling_random(c['coords'][0], c['voxel'], [c['levels'][li]], c['add_rnd3d'],
+                                                      shifts=[c['shifts'][li]], uniforms=[c['uniforms'][li]])
+        assert not np.array_equal(kp[0][:, 0], c['kp'][li]), tag
+    c = graph.random_golden_case(g, 'arr')
+    assert isinstance(c['voxel'], np.ndarray) and c['voxel'].shape == (3,)
+    _, kp = graph.multi_layer_downsampling_random(c['xyz'], float(c['voxel'][0]), c['levels'],
+                                                  uniforms=c['uniforms'])
+    assert len(kp[0]) != len(c['kp'][0])
+
+
+def _cap_fixture():
+    """Radius graph with a long row (dst 0: 6 members), a short one (dst 1: 2), one of exactly the cap (dst 2: 3),
+    an empty one (dst 3) and another long one (dst 4: 4); cap 3."""
+    full = np.array([[s, 0] for s in (1, 2, 4, 5, 7, 9)] + [[3, 1], [8, 1]] + [[0, 2], [6, 2], [9, 2]] +
+                    [[2, 4], [3, 4], [5, 4], [6, 4]], dtype=np.int64)
+    capped = np.array([[2, 0], [5, 0], [9, 0], [3, 1], [8, 1], [0, 2], [6, 2], [9, 2], [2, 4], [3, 4], [6, 4]],
+                      dtype=np.int64)
+    return full, capped
+
+
+def test_check_neighbor_cap_accepts_a_valid_cap():
+    full, capped = _cap_fixture()
+    assert graph.check_neighbor_cap(full, capped, 3) == 2
+    other = capped.copy()
+    other[:3, 0] = (1, 4, 7)                   # any other subset of the long row is as valid
+    assert graph.check_neighbor_cap(full, other, 3) == 2
+    assert graph.check_neighbor_cap(full, full, 6) == 0
+
+
+@pytest.mark.parametrize('breakage', ['duplicate', 'outside', 'short_row', 'long_short', 'long_long', 'exact_row',
+                                      'moved_dst'])
+def test_check_neighbor_cap_rejects_a_broken_cap(breakage):
+    """The checker behind the neighbour-cap GPU tests must be able to fail."""
+    full, capped = _cap_fixture()
+    bad = capped.copy()
+    if breakage == 'duplicate':                # a long row keeps one member twice
+        bad[1, 0] = bad[0, 0]
+    elif breakage == 'outside':                # a long row keeps a point that is not its neighbour
+        bad[1, 0] = 3
+    elif breakage == 'short_row':              # a short row loses a member for a neighbour of another row
+        bad[3, 0] = 6
+    elif breakage == 'long_short':             # a long row keeps cap - 1 members
+        bad = np.delete(bad, 0, axis=0)
+    elif breakage == 'long_long':              # a long row keeps cap + 1 members
+        bad = np.vstack([bad, [[1, 0]]])
+    elif breakage == 'exact_row':              # a row of exactly the cap loses a member
+        bad = np.delete(bad, 6, axis=0)
+    else:                                      # an edge changes rows
+        bad[10, 1] = 0
+    with pytest.raises(AssertionError):
+        graph.check_neighbor_cap(full, bad, 3)

@@ -174,12 +174,90 @@ def kitti_goldens():
     print('kitti: points in image', pts.xyz.shape, 'result lines', text.count('\n') - 1)
 
 
+def _with_recorded_draws(fn, shifts, uniforms):
+    """Call fn() - which runs the reference's multi_layer_downsampling_random - with its two random sources patched to
+    recorded numbers.  The level a draw belongs to is read from the reference's own loop: li = the number of levels it
+    has finished (len(keypoint_indices_list)).  np.random.random((1, 3)) -> shifts[li]; random.choice(seq) for the o-th
+    voxel of level li -> seq[floor(uniforms[li][o] * len(seq))].  -> (fn(), {li: number of voxels drawn})."""
+    import random as _random
+    drawn = {}
+
+    def level_of_caller():
+        return len(sys._getframe(2).f_locals['keypoint_indices_list'])
+
+    def fake_choice(seq):
+        li = level_of_caller()
+        o = drawn.get(li, 0)
+        drawn[li] = o + 1
+        return seq[min(int(np.float32(uniforms[li][o]) * np.float32(len(seq))), len(seq) - 1)]
+
+    def fake_random(size=None):
+        assert size == (1, 3)
+        return np.array(shifts[level_of_caller()], dtype=np.float64).reshape(1, 3)
+
+    orig_choice, orig_rand = _random.choice, np.random.random
+    _random.choice, np.random.random = fake_choice, fake_random
+    try:
+        return fn(), drawn
+    finally:
+        _random.choice, np.random.random = orig_choice, orig_rand
+
+
+def _floor_divide_boundary_pairs(xyz, voxel):
+    """Two points per axis that the float32 and the float64 voxel rule partition differently.  A sits where
+    floor_divide(p - min, voxel) in float32 and in float64 disagree on that axis (float32(0.8) > 0.8, so e.g.
+    min + 29.6f is voxel 36 in float32 and 37 in float64), B in the middle of the higher of the two voxels; on the other
+    two axes both sit in the middle of a voxel beyond the cloud.  One rule puts A and B in one voxel, the other in two."""
+    mn, mx = xyz.min(axis=0), xyz.max(axis=0)
+    v32 = np.float32(voxel)
+    pairs = []
+    for a in range(3):
+        found = None
+        for k in range(20, 400):
+            c = np.float32(mn[a] + k * voxel)
+            for step in range(-8, 9):
+                p = (c.view(np.int32) + np.int32(step)).view(np.float32)
+                d = np.float32(p - mn[a])
+                i32, i64 = int(np.floor_divide(d, v32)), int(np.floor_divide(np.float64(d), voxel))
+                if i32 != i64:
+                    found = (p, max(i32, i64))
+                    break
+            if found:
+                break
+        assert found, 'no float32/float64 floor-divide disagreement on axis %d' % a
+        p, hi = found
+        pt = np.empty(3, dtype=np.float32)
+        for b in range(3):
+            if b != a:         # a voxel of its own beyond the cloud, different for every axis' pair
+                pt[b] = np.float32(mn[b] + (np.floor((mx[b] - mn[b]) / voxel) + 3 + 2 * a + 0.5) * voxel)
+        pt_a, pt_b = pt.copy(), pt.copy()
+        pt_a[a] = p
+        pt_b[a] = np.float32(mn[a] + (hi + 0.5) * voxel)
+        pairs += [pt_a, pt_b]
+    return np.asarray(pairs, dtype=np.float32)
+
+
+RANDOM_LEVEL_CONFIGS = [   # the structure of configs/*_train_config without the neighbour cap, so edges are exact
+    {'graph_gen_kwargs': {'num_neighbors': -1, 'radius': 1.0}, 'graph_gen_method': 'disjointed_rnn_local_graph_v3',
+     'graph_level': 0, 'graph_scale': 1},
+    {'graph_gen_kwargs': {'num_neighbors': -1, 'radius': 4.0}, 'graph_gen_method': 'disjointed_rnn_local_graph_v3',
+     'graph_level': 1, 'graph_scale': 1}]
+
+
 def graph_random_goldens():
     """tests/golden/graph_random.npz: the reference's OWN multi_layer_downsampling_random (graph_gen.py:92-153) with its
-    two random sources patched to recorded numbers: np.random.random -> `shift`, random.choice(seq) ->
-    seq[floor(u[o] * len(seq))] for the o-th call.  The CUDA path gets the same numbers as arguments and must return
-    the same keypoints, with and without add_rnd3d."""
-    import random as _random
+    two random sources patched to recorded numbers (_with_recorded_draws): one grid shift and one uniform array per new
+    scale, the uniforms indexed by voxel rank in first-appearance order, which is how the CUDA path consumes them.  The
+    CUDA path gets the same numbers as arguments and must return the same keypoints.
+
+    * ``plain`` / ``rnd3d``: levels [1, 1], scalar voxel 0.8, without / with add_rnd3d (keys <kind>_<tag>).
+    * ``ms_plain`` / ``ms_rnd3d``: levels [1, 2, 2]: the second scale voxelises level 1's vertices on the grid of the
+      ORIGINAL cloud's minimum (:107-110, 123-128), which differs from level 1's own minimum here.
+    * ``arr``: voxel np.array([0.8] * 3) through gen_multi_level_local_graph_v3(downsample_method='random') with
+      num_neighbors -1, on a cloud with points where float32 and float64 floor-division disagree: an array voxel size
+      divides in float64 (:123-124), a scalar one in float32.  The edge lists are the reference's ball tree, canonical.
+    Cases after the first two: keys <kind>_<tag>_<level index>; levels_<tag>, voxel_<tag>, add_<tag>, radii_<tag> with
+    the edge lists, and xyz_<tag> where the cloud is not ``xyz``.  oracle.graph.random_golden_case reads them back."""
     ref = reference_graph.load()
     xyz, _ = synth.lidar_frame(3, 8000)
     rng = np.random.default_rng(0)
@@ -187,20 +265,8 @@ def graph_random_goldens():
     for add in (False, True):
         shift = rng.random((1, 3))
         u = rng.random(len(xyz)).astype(np.float32)
-        counter = {'o': 0}
-
-        def fake_choice(seq):
-            o = counter['o']
-            counter['o'] += 1
-            return seq[min(int(np.float32(u[o]) * np.float32(len(seq))), len(seq) - 1)]
-
-        orig_choice, orig_rand = _random.choice, np.random.random
-        _random.choice = fake_choice
-        np.random.random = lambda size=None: shift.copy()
-        try:
-            vc, kp = ref.multi_layer_downsampling_random(xyz, 0.8, [1, 1], add_rnd3d=add)
-        finally:
-            _random.choice, np.random.random = orig_choice, orig_rand
+        (vc, kp), _ = _with_recorded_draws(lambda: ref.multi_layer_downsampling_random(xyz, 0.8, [1, 1], add_rnd3d=add),
+                                           [shift, None], [u, None])
         tag = 'rnd3d' if add else 'plain'
         out['shift_' + tag] = shift
         out['u_' + tag] = u
@@ -209,6 +275,64 @@ def graph_random_goldens():
                                                          uniforms=[u, None])
         assert np.array_equal(kp[0], kp2[0]) and np.array_equal(vc[1], vc2[1]), 'oracle restatement != reference'
         print('graph_random', tag, 'keypoints', len(kp[0]))
+
+    rng = np.random.default_rng(2)      # a draw for which level 1's minimum differs from the cloud's in both cases
+    cases = []
+    levels = [1, 2, 2]
+    for add in (False, True):
+        tag = 'ms_rnd3d' if add else 'ms_plain'
+        shifts = [rng.random((1, 3)), rng.random((1, 3)), None]
+        uniforms = [rng.random(len(xyz)).astype(np.float32), rng.random(len(xyz)).astype(np.float32), None]
+        (vc, kp), drawn = _with_recorded_draws(
+            lambda: ref.multi_layer_downsampling_random(xyz, 0.8, levels, add_rnd3d=add), shifts, uniforms)
+        uniforms[1] = uniforms[1][:len(vc[1])]         # one per point of the level it voxelises
+        vo, ko = graph.multi_layer_downsampling_random(xyz, 0.8, levels, add_rnd3d=add, shifts=shifts, uniforms=uniforms)
+        for li in range(len(levels)):
+            assert np.array_equal(kp[li], ko[li]) and np.array_equal(vc[li + 1], vo[li + 1]), 'oracle != reference'
+        # the fixture tells the grid origins apart: level 1's own minimum partitions level 2 differently
+        _, k_own = graph.multi_layer_downsampling_random(vc[1], 0.8, [2], add_rnd3d=add, shifts=[shifts[1]],
+                                                         uniforms=[uniforms[1]])
+        assert not np.array_equal(k_own[0], kp[1]), 'the second scale does not depend on the grid origin'
+        cases.append((tag, xyz, levels, np.float64(0.8), add, shifts, uniforms, vc, kp, None))
+        print('graph_random', tag, 'keypoints', [len(k) for k in kp], 'voxels drawn', drawn)
+
+    cloud, _ = synth.lidar_frame(5, 3000)
+    cloud = np.vstack([cloud, _floor_divide_boundary_pairs(cloud, 0.8)])
+    voxel = np.array([0.8, 0.8, 0.8])
+    u = rng.random(len(cloud)).astype(np.float32)
+    (vc, kp, edges), _ = _with_recorded_draws(
+        lambda: ref.gen_multi_level_local_graph_v3(cloud, voxel, RANDOM_LEVEL_CONFIGS, downsample_method='random'),
+        [None, None], [u, None])
+    (_, kp_scalar), _ = _with_recorded_draws(lambda: ref.multi_layer_downsampling_random(cloud, 0.8, [1, 1]),
+                                             [None, None], [u, None])
+    assert len(kp_scalar[0]) != len(kp[0]), 'array and scalar voxel sizes partition this cloud alike'
+    vo, ko = graph.multi_layer_downsampling_random(cloud, voxel, [1, 1], shifts=[None, None], uniforms=[u, None])
+    edges = [graph.canonical_edges(e) for e in edges]
+    for li in range(2):
+        assert np.array_equal(kp[li], ko[li]) and np.array_equal(vc[li + 1], vo[li + 1]), 'oracle != reference'
+        cfg = RANDOM_LEVEL_CONFIGS[li]
+        assert np.array_equal(edges[li], graph.radius_graph(vo[li], vo[li + 1], cfg['graph_gen_kwargs']['radius']))
+    cases.append(('arr', cloud, [1, 1], voxel, False, [None, None], [u, None], vc, kp, edges))
+    print('graph_random arr keypoints', len(kp[0]), 'with a scalar voxel', len(kp_scalar[0]))
+
+    for tag, pts, lv, vox, add, shifts, uniforms, vc, kp, edges in cases:
+        if pts is not xyz:
+            out['xyz_' + tag] = pts
+        out['levels_' + tag] = np.asarray(lv, dtype=np.float64)
+        out['voxel_' + tag] = np.asarray(vox, dtype=np.float64)
+        out['add_' + tag] = np.bool_(add)
+        for li in range(len(lv)):
+            if shifts[li] is not None and add:
+                out['shift_%s_%d' % (tag, li)] = shifts[li]
+            if uniforms[li] is not None:
+                out['u_%s_%d' % (tag, li)] = uniforms[li]
+            out['kp_%s_%d' % (tag, li)] = np.asarray(kp[li])[:, 0].astype(np.int32)
+            out['coords_%s_%d' % (tag, li + 1)] = np.asarray(vc[li + 1], dtype=np.float32)
+        for lvl, e in enumerate(edges or []):
+            out['edges_%s_%d' % (tag, lvl)] = e.astype(np.int32)
+        if edges:
+            out['radii_' + tag] = np.array([c['graph_gen_kwargs']['radius'] for c in RANDOM_LEVEL_CONFIGS])
+    out['cases'] = np.array([c[0] for c in cases])
     np.savez_compressed(os.path.join(GOLDEN, 'graph_random.npz'), **out)
 
 
